@@ -75,6 +75,51 @@ def tsdf_algorithmic_bytes(blocks, color, width=640, height=480):
     return blocks * 4096 * 2 * s_vox + width * height * 2 + (width * height * 3 if color else 0) + blocks * 16 + touch
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE_BLOCKS = 128
+
+
+def volume_outputs(L, v, stream, torch, prefix, color):
+    """What a caller of the TSDF path receives: the key of every active block (sorted, since the hash map's slot order
+    depends on insertion timing) and tsdf / weight (/ colour) of a fixed, seeded sample of those blocks."""
+    from open3d_b200.t._libshim import device_view
+    torch.cuda.synchronize()
+    size = L.check(L.lib.o3db_vbg_size(v, stream))
+    cap = L.lib.o3db_vbg_capacity(v)
+    idx = torch.empty(size, dtype=torch.int32, device="cuda")
+    L.check(L.lib.o3db_vbg_active_indices(v, idx.data_ptr(), size, stream))
+    idx = idx.long()
+    keys = device_view(L.lib.o3db_vbg_key_buffer(v), (cap, 3), torch.int32)[idx].cpu().numpy()
+    order = np.lexsort((keys[:, 2], keys[:, 1], keys[:, 0]))
+    pick = np.sort(np.random.default_rng(0).choice(size, min(size, DUMP_SAMPLE_BLOCKS), replace=False))
+    slots = idx[torch.from_numpy(order[pick]).cuda()]
+    vox = RES ** 3
+    out = {f"{prefix}_block_keys": keys[order].astype(np.float64),
+           f"{prefix}_sample_block_keys": keys[order[pick]].astype(np.float64),
+           f"{prefix}_sample_tsdf": device_view(L.lib.o3db_vbg_tsdf_buffer(v), (cap, vox), torch.float32)[slots],
+           f"{prefix}_sample_weight": device_view(L.lib.o3db_vbg_weight_buffer(v), (cap, vox), torch.uint16)
+           .view(torch.int16)[slots].int().bitwise_and(0xFFFF).float()}
+    if color:
+        out[f"{prefix}_sample_color"] = device_view(L.lib.o3db_vbg_color_buffer(v), (cap, vox, 3), torch.uint16) \
+            .view(torch.int16)[slots].int().bitwise_and(0xFFFF).float()
+    return out
+
+
+def write_outputs(dirname, arrays):
+    """--dump-outputs: one DIR/<name>.npy per array; doubles and integers as float64, everything else as float32."""
+    os.makedirs(dirname, exist_ok=True)
+    conv = {}
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if hasattr(a, "cpu") else np.asarray(a)
+        exact64 = a.dtype == np.float64 or (a.dtype.kind in "iu" and a.dtype.itemsize > 2)
+        conv[name] = np.ascontiguousarray(a, np.float64 if exact64 else np.float32)
+    total = sum(a.nbytes for a in conv.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    for name, a in conv.items():
+        np.save(os.path.join(dirname, f"{name}.npy"), a)
+
+
 class ClockSampler:
     """Samples SM clocks / throttle reasons during the timed region (B200_PROFILING.md): NVML in-process
     every 5 ms (the timed region is tens of milliseconds), nvidia-smi as a fallback."""
@@ -445,6 +490,9 @@ def main():
                     help="also run BASELINE configs[3] once (multi-scale ColoredICP, 3 scales, 5M points, source split over the "
                          "ranks); always on for N > 1")
     ap.add_argument("--config3-points", type=int, default=5_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step of each timed path returned to its caller "
+                         "as DIR/<name>.npy (the inputs are seeded: two builds can be compared output for output)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -553,6 +601,10 @@ def main():
                 "avg_launch_us": kern_ms * 1e3, "peak_source": peak_src}
     final = {"fitness": res.fitness, "inlier_rmse": res.inlier_rmse, "num_iterations": res.num_iterations,
              "transformation_error_vs_ground_truth": float(np.abs(np.array(res.transformation).reshape(4, 4) - T_gt).max())}
+    dump = {"icp_transformation": np.array(res.transformation).reshape(4, 4),
+            "icp_fitness": np.float64([res.fitness]), "icp_inlier_rmse": np.float64([res.inlier_rmse]),
+            "icp_num_iterations": np.float64([res.num_iterations]),
+            "icp_num_correspondences": np.float64([res.num_correspondences])}
     L.lib.o3db_icp_destroy(h)
 
     # e2e: host buffers (pinned) through the C ABI, everything inside the timed region
@@ -644,7 +696,8 @@ def main():
     # ----------------------------------------------------------------- TSDF
     tsdf = None
     if not args.skip_tsdf:
-        tsdf = bench_tsdf(args, rank, world, local_rank, L, torch, stream, barrier, max_over_ranks, peak, peak_src)
+        tsdf = bench_tsdf(args, rank, world, local_rank, L, torch, stream, barrier, max_over_ranks, peak, peak_src,
+                          dump if args.dump_outputs else None)
 
     # ---------------------------------------------------------- CPU baseline
     cpu = None
@@ -682,13 +735,17 @@ def main():
                     "dense_slam": tsdf.get("dense_slam"), "icp": icp_line}
         else:
             line = dict(icp_line, tsdf=tsdf)
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, dump)
         print(json.dumps(line), flush=True)
     if world > 1:
         comm.close()
         dist.destroy_process_group()
 
 
-def bench_tsdf(args, rank, world, local_rank, L, torch, stream, barrier, max_over_ranks, peak, peak_src):
+def bench_tsdf(args, rank, world, local_rank, L, torch, stream, barrier, max_over_ranks, peak, peak_src, dump=None):
+    """`dump` (a dict, or None): receives the volume of the last timed device pass of each variant, the last ray cast
+    and the dense-SLAM loop's final pose."""
     from tests.synth import PRIMESENSE_K, camera_pose, render_depth
     F = args.tsdf_frames
     mine = list(range(rank, F, world))                      # frames round-robin over independent volumes
@@ -756,6 +813,8 @@ def bench_tsdf(args, rank, world, local_rank, L, torch, stream, barrier, max_ove
                         L.check(L.lib.o3db_vbg_exec_stats(v, C.byref(em), C.byref(el), 1, stream))
                         exec_ms += em.value
                         exec_launches += el.value
+                        if dump is not None and rank == 0 and it == warmup + steps - 1:
+                            dump.update(volume_outputs(L, v, stream, torch, f"tsdf_{name}", color))
                 if profiled:
                     if True:
                         tm, im, nf = C.c_double(0), C.c_double(0), C.c_int64(0)
@@ -843,6 +902,8 @@ def bench_tsdf(args, rank, world, local_rank, L, torch, stream, barrier, max_ove
         b.record()
         torch.cuda.synchronize()
         ms = a.elapsed_time(b) / reps
+        if dump is not None:
+            dump.update(raycast_depth=rd.clone(), raycast_color=rc.clone())
         out["raycast"] = {"workload": "slam::Model::SynthesizeModelFrame 640x480 depth+color after 60 fused frames",
                           "ms_per_frame": ms, "frames_per_sec": 1e3 / ms, "rays_per_sec": 640 * 480 / (ms * 1e-3),
                           "hit_fraction": float((rd > 0).float().mean()), "gpu_launches_per_frame":
@@ -905,6 +966,8 @@ def bench_tsdf(args, rank, world, local_rank, L, torch, stream, barrier, max_ove
     if max_over_ranks(1.0 if slam_err else 0.0) > 0 and not slam_err:
         slam_err = "tracking failed on another rank"      # its clock is meaningless: report, never average over it
     gt = camera_pose(seg[-1], n_frames=F)
+    if dump is not None and rank == 0 and not slam_err:
+        dump["dense_slam_final_pose"] = pose
     out["dense_slam"] = {"error": slam_err} if slam_err else {"workload": "slam::Model loop (odometry PointToPlane {6,3,1} + integrate + ray cast), "
                                      f"{S} consecutive 640x480 RGB-D frames per GPU, poses estimated",
                          "baseline_config": "configs[4] (bounded segment)", "frames_per_sec": world * S / (slam_ms * 1e-3),

@@ -251,7 +251,7 @@ def test_config3_colored_multiscale_icp_3_scales_500k_vs_oracle(o3d):
 
 # ------------------------------------------------------------------ §8(e)
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_sharded_icp_equals_single_gpu_on_2_gpus():
     """tests/multigpu_check.py under torchrun, 2 ranks over NCCL: source-sharded point-to-plane ICP and ColoredICP
     (one 30-double all-reduce per iteration inside the library) == the single-GPU run on the whole source."""

@@ -18,7 +18,7 @@ from tests.synth import PRIMESENSE_K, camera_pose, make_colors, make_icp_pair, r
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SO = os.path.join(ROOT, "integration", "_build", "libo3d_forwarders.so")
-needs_so = pytest.mark.skipif(not os.path.exists(SO), reason="integration/_build not built (needs /root/reference at build time)")
+needs_so = pytest.mark.skipif(not os.path.exists(SO), reason="integration/_build not built (needs the Open3D sources at build time)")
 
 REFERENCE_SYMBOLS = [   # demangled prefixes the reference's callers link against
     "open3d::t::pipelines::kernel::ComputePosePointToPlaneCUDA(",

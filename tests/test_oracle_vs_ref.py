@@ -1,161 +1,64 @@
-"""Validate the CPU oracle against the REAL reference code: oracle/_ref/libo3dref.so holds
-functions compiled straight from Open3D's own headers (oracle/ref_shim/ref_shim.cpp lists
-them with file:line).  Every comparison here is bit-exact.  CPU only."""
-import ctypes as C
-import os
-
+"""Validate the CPU oracle against the REAL reference code: the outputs of functions compiled straight from Open3D's
+own headers (oracle/ref_shim/ref_shim.cpp lists them with file:line), stored in tests/golden/ref_oracle_vs_ref.npz by
+tests/golden/make_ref_vectors.py from the inputs built here.  Every comparison is bit-exact unless its docstring says
+otherwise.  CPU only."""
 import numpy as np
 import pytest
 
 import oracle
+from tests.ref_vectors import Vectors
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "oracle", "_ref", "libo3dref.so")
-
-pytestmark = pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref not built (needs /root/reference)")
-
-f32p, f64p, i64p, i32p = (C.POINTER(t) for t in (C.c_float, C.c_double, C.c_int64, C.c_int))
+ROBUST_RS = (0.98, -0.37, 1e-4, 2.5, -7.0, 0.0311)
+ROBUST_SCALES = (1.0, 0.05, 3.0)
+ROBUST_SHAPES = (1.0, 2.0, 2.0015, 1.9975, 0.0, 0.0005, -2.0, -1e8, 0.5)
+BOUNDARY_POINTS = [(0, 0), (639, 479), (639.0001, 10), (-0.0, 5), (-1e-7, 5), (10, 479.5), (np.nan, 1)]
+ROBUST = [("L2Loss", 1.0, 1.0), ("L1Loss", 1.0, 1.0), ("HuberLoss", 0.01, 1.0), ("TukeyLoss", 0.03, 1.0),
+          ("GeneralizedLoss", 0.5, 1.3)]
+HUBER_DELTAS = (0.05, 0.1, 1.2)
 
 
 @pytest.fixture(scope="module")
 def ref():
-    L = C.CDLL(REF)
-    L.ref_spatial_hash.restype = C.c_uint64
-    L.ref_spatial_hash.argtypes = [C.c_int] * 3
-    L.ref_minivec_hash_i32x3.restype = C.c_uint64
-    L.ref_minivec_hash_i32x3.argtypes = [C.c_int] * 3
-    L.ref_robust_weight_f64.restype = C.c_double
-    L.ref_robust_weight_f64.argtypes = [C.c_int, C.c_double, C.c_double, C.c_double]
-    L.ref_robust_weight_f32.restype = C.c_float
-    L.ref_robust_weight_f32.argtypes = [C.c_int, C.c_double, C.c_double, C.c_float]
-    L.ref_jacobian_p2plane_f32.argtypes = [C.c_int64, f32p, f32p, f32p, i64p, f32p, f32p]
-    L.ref_jacobian_colored_f32.argtypes = [C.c_int64] + [f32p] * 6 + [i64p, C.c_float, C.c_float, f32p, f32p, f32p, f32p]
-    L.ref_pose_to_transformation.argtypes = [f64p, f64p]
-    L.ref_transform_points_f32.argtypes = [f32p, f32p, C.c_int64]
-    L.ref_transform_normals_f32.argtypes = [f32p, f32p, C.c_int64]
-    L.ref_compute_voxel_index_f32.argtypes = [f32p, C.c_float, i32p]
-    L.ref_transform_indexer.argtypes = [f64p, f64p, C.c_float, C.c_int, f32p, f32p]
-    L.ref_workload_to_coord3.argtypes = [C.c_int, C.c_int, i32p]
-    L.ref_in_boundary2.argtypes = [C.c_int, C.c_int, C.c_float, C.c_float]
-    return L
+    return Vectors("oracle_vs_ref")
 
 
-def _p(a, t):
-    return a.ctypes.data_as(t)
+# ------------------------------------------------ inputs (shared with tests/golden/make_ref_vectors.py)
 
-
-def test_hashes(ref):
+def hash_inputs():
     rng = np.random.default_rng(0)
     keys = rng.integers(-2**31, 2**31 - 1, (500, 3), dtype=np.int64).astype(np.int32)
     keys[:3] = [[0, 0, 0], [-1, 3, 2], [2**31 - 1, -2**31, 5]]
-    want = [ref.ref_minivec_hash_i32x3(*map(int, k)) for k in keys]
-    assert oracle.minivec_hash(keys).tolist() == want
     cells = rng.integers(-100000, 100000, (500, 3)).astype(np.int32)
-    assert oracle.spatial_hash(cells).tolist() == [ref.ref_spatial_hash(*map(int, c)) for c in cells]
-    for p, inv in [((-0.05, 0.149, 0.1), 10.0), ((3.7, -2.2, 0.0), 7.5), ((1e-8, -1e-8, 5.0), 10.0)]:
-        a = np.array(p, np.float32)
-        out = np.zeros(3, np.int32)
-        ref.ref_compute_voxel_index_f32(_p(a, f32p), inv, _p(out, i32p))
-        assert oracle.compute_voxel_index(a, inv).tolist() == out.tolist()
+    points = [((-0.05, 0.149, 0.1), 10.0), ((3.7, -2.2, 0.0), 7.5), ((1e-8, -1e-8, 5.0), 10.0)]
+    return keys, cells, points
 
 
-def test_robust_kernel_weights_bit_exact(ref):
-    rs = [0.98, -0.37, 1e-4, 2.5, -7.0, 0.0311]
-    for method in range(7):
-        for scale in (1.0, 0.05, 3.0):
-            for shape in (1.0, 2.0, 2.0015, 1.9975, 0.0, 0.0005, -2.0, -1e8, 0.5):
-                for r in rs:
-                    assert oracle.robust_weight(method, scale, shape, r) == ref.ref_robust_weight_f64(method, scale, shape, r)
-                    a = oracle.robust_weight(method, scale, shape, r, f32=True)
-                    b = ref.ref_robust_weight_f32(method, scale, shape, r)
-                    assert np.float32(a).tobytes() == np.float32(b).tobytes(), (method, scale, shape, r, a, b)
-
-
-def test_jacobian_and_sums_bit_exact(ref):
+def p2plane_inputs():
     from tests.synth import make_icp_pair
     src, tgt, nrm, _ = make_icp_pair(3000, seed=21)
     idx, _, _ = oracle.hybrid_search(tgt, src, 0.05, 1)
-    corr = np.ascontiguousarray(idx[:, 0].astype(np.int64))
-    # re-accumulate the 29 sums in f32, in index order, from the REFERENCE's Jacobian function
-    acc = np.zeros(29, np.float32)
-    J = np.zeros(6, np.float32)
-    r = C.c_float(0)
-    for i in range(len(src)):
-        if not ref.ref_jacobian_p2plane_f32(i, _p(src, f32p), _p(tgt, f32p), _p(nrm, f32p), _p(corr, i64p), _p(J, f32p), C.byref(r)):
-            continue
-        rr = np.float32(r.value)
-        s = 0
-        for j in range(6):
-            for k in range(j + 1):
-                acc[s] += J[j] * np.float32(1.0) * J[k]
-                s += 1
-            acc[21 + j] += J[j] * np.float32(1.0) * rr
-        acc[27] += rr
-        acc[28] += np.float32(1)
-    got = oracle.pose_p2plane_sums(src, tgt, nrm, corr)["sums32"]
-    assert got.tobytes() == acc.tobytes()
+    return src, tgt, nrm, np.ascontiguousarray(idx[:, 0].astype(np.int64))
 
 
-def test_colored_jacobian_bit_exact(ref):
+def colored_inputs():
     from tests.synth import make_colors, make_icp_pair
     src, tgt, nrm, _ = make_icp_pair(400, seed=22)
     sc, tc = make_colors(src), make_colors(tgt)
     grad = np.random.default_rng(1).normal(0, 0.5, tgt.shape).astype(np.float32)
     idx, _, _ = oracle.hybrid_search(tgt, src, 0.05, 1)
-    corr = np.ascontiguousarray(idx[:, 0].astype(np.int64))
-    lam = 0.968
-    slg, slp = np.float32(np.sqrt(lam)), np.float32(np.sqrt(1.0 - lam))
-    acc = np.zeros(29, np.float64)
-    JG, JI = np.zeros(6, np.float32), np.zeros(6, np.float32)
-    rG, rI = C.c_float(0), C.c_float(0)
-    one = np.float32(1)
-    for i in range(len(src)):
-        ok = ref.ref_jacobian_colored_f32(i, _p(src, f32p), _p(sc, f32p), _p(tgt, f32p), _p(nrm, f32p), _p(tc, f32p),
-                                          _p(grad, f32p), _p(corr, i64p), float(slg), float(slp), _p(JG, f32p),
-                                          _p(JI, f32p), C.byref(rG), C.byref(rI))
-        if not ok:
-            continue
-        g, q = np.float32(rG.value), np.float32(rI.value)
-        s = 0
-        for j in range(6):
-            for k in range(j + 1):
-                acc[s] += np.float32(JG[j] * one * JG[k] + JI[j] * one * JI[k])
-                s += 1
-            acc[21 + j] += np.float32(JG[j] * one * g + JI[j] * one * q)
-        acc[27] += np.float32(g * g + q * q)
-        acc[28] += 1
-    got = oracle.pose_colored_sums(src, sc, tgt, nrm, tc, grad, corr, lam)["sums64"]
-    assert np.array_equal(got, acc)
+    return src, sc, tgt, nrm, tc, grad, np.ascontiguousarray(idx[:, 0].astype(np.int64)), 0.968
 
 
-def test_pose_transform_and_indexers_bit_exact(ref):
+def pose_inputs():
     rng = np.random.default_rng(3)
-    for _ in range(20):
-        pose = rng.normal(0, 0.3, 6)
-        T = np.zeros(16)
-        ref.ref_pose_to_transformation(_p(pose, f64p), _p(T, f64p))
-        assert np.array_equal(oracle.pose_to_transformation(pose).ravel(), T)
+    poses = np.stack([rng.normal(0, 0.3, 6) for _ in range(20)])
     T = oracle.pose_to_transformation(np.array([0.2, -0.1, 0.4, 1.0, -2.0, 0.5]))
     pts = rng.uniform(-4, 4, (999, 3)).astype(np.float32)
-    Tf = np.ascontiguousarray(T.astype(np.float32))
-    a, b = pts.copy(), pts.copy()
-    ref.ref_transform_points_f32(_p(Tf, f32p), _p(a, f32p), len(a))
-    ref.ref_transform_normals_f32(_p(Tf, f32p), _p(b, f32p), len(b))
-    assert oracle.transform_points(T, pts).tobytes() == a.tobytes()
-    assert oracle.transform_normals(T, pts).tobytes() == b.tobytes()
-    # ArrayIndexer conventions the TSDF oracle relies on
-    out = np.zeros(3, np.int32)
-    for res in (2, 8, 16):
-        for w in range(0, res ** 3, 7):
-            ref.ref_workload_to_coord3(res, w, _p(out, i32p))
-            assert out.tolist() == [w % res, (w // res) % res, w // (res * res)]
-    for x, y in [(0, 0), (639, 479), (639.0001, 10), (-0.0, 5), (-1e-7, 5), (10, 479.5), (np.nan, 1)]:
-        want = bool(y >= 0 and x >= 0 and y <= 480 - 1.0 and x <= 640 - 1.0)
-        assert bool(ref.ref_in_boundary2(480, 640, x, y)) == want
+    return poses, T, pts
 
 
-def test_tsdf_geometry_against_transform_indexer(ref):
-    """One voxel of oracle.tsdf_integrate re-derived with the reference's TransformIndexer."""
+def tsdf_geometry_inputs():
+    """One frame fused by the oracle, and 300 (block, voxel, voxel position) samples of it."""
     from tests.synth import PRIMESENSE_K, camera_pose, render_depth
     T = camera_pose(17)
     E = oracle.inverse_transformation(T)
@@ -165,39 +68,19 @@ def test_tsdf_geometry_against_transform_indexer(ref):
     tsdf = np.zeros((cap, 4096), np.float32)
     wt = np.zeros((cap, 4096), np.uint16)
     oracle.tsdf_integrate(depth, None, np.arange(cap, dtype=np.int32), keys, tsdf, wt, None, PRIMESENSE_K, PRIMESENSE_K, E)
-    K = np.ascontiguousarray(PRIMESENSE_K)
-    Ec = np.ascontiguousarray(E)
     rng = np.random.default_rng(5)
-    checked = 0
-    trunc = np.float32(0.008) * np.float32(8.0)
+    samples = []
     for b in rng.integers(0, cap, 300):
         v = int(rng.integers(0, 4096))
         xv, yv, zv = v % 16, (v // 16) % 16, v // 256
         vin = np.array([keys[b][0] * 16 + xv, keys[b][1] * 16 + yv, keys[b][2] * 16 + zv], np.float32)
-        cam, uv = np.zeros(3, np.float32), np.zeros(3, np.float32)
-        ref.ref_transform_indexer(_p(K, f64p), _p(Ec, f64p), 0.008, 0, _p(vin, f32p), _p(cam, f32p))
-        ref.ref_transform_indexer(_p(K, f64p), _p(Ec, f64p), 0.008, 1, _p(cam, f32p), _p(uv, f32p))
-        u, vv = uv[0], uv[1]
-        if not ref.ref_in_boundary2(480, 640, float(u), float(vv)):
-            assert wt[b, v] == 0
-            continue
-        d = np.float32(depth[int(vv), int(u)]) / np.float32(1000.0)
-        sdf = np.float32(d - cam[2])
-        if d <= 0 or d > 3.0 or cam[2] <= 0 or sdf < -trunc:
-            assert wt[b, v] == 0
-            continue
-        sdf = np.float32(min(sdf, trunc)) / trunc
-        assert wt[b, v] == 1 and np.float32(tsdf[b, v]).tobytes() == np.float32((np.float32(0) * np.float32(0) + sdf) * np.float32(1.0)).tobytes()
-        checked += 1
-    assert checked > 50
+        samples.append((int(b), v, vin))
+    return np.ascontiguousarray(PRIMESENSE_K), np.ascontiguousarray(E), depth, tsdf, wt, samples
 
 
-def test_svd3_solver_bit_exact_vs_reference(ref):
-    """oracle/svd3_oracle.c (svd3x3<float> + solve_svd3x3<float> restated, indexed by axis triples) vs the
-    reference's own solve_svd3x3<float> (core/linalg/kernel/SVD3x3.h:2170-2215) compiled unmodified in oracle/_ref:
-    identical BYTES on general, symmetric-PSD, colour-gradient-like (condition ~1e5), diagonal/scaled, rank-1
-    single-entry and all-zero systems — every branch of the approximate Givens, the column sort and the QR."""
-    ref.ref_solve_svd3x3_f32.argtypes = [f32p, f32p, f32p]
+def svd3_systems():
+    """6000 (kind, A, b) f32 systems: general, symmetric-PSD, colour-gradient-like (condition ~1e5), diagonal/scaled,
+    rank-1 single-entry and all-zero."""
     rng = np.random.default_rng(0)
     for t in range(6000):
         kind = t % 6
@@ -219,12 +102,157 @@ def test_svd3_solver_bit_exact_vs_reference(ref):
             A[rng.integers(0, 3), rng.integers(0, 3)] = rng.standard_normal()
         else:
             A = np.zeros((3, 3))
-        A32 = np.ascontiguousarray(A, np.float32).reshape(9)
-        b32 = rng.standard_normal(3).astype(np.float32)
-        want = np.zeros(3, np.float32)
-        ref.ref_solve_svd3x3_f32(_p(A32, f32p), _p(b32, f32p), _p(want, f32p))
-        got = oracle.solve_svd3x3(A32, b32)
-        assert got.tobytes() == want.tobytes(), (kind, A32, b32, got, want)
+        yield kind, np.ascontiguousarray(A, np.float32).reshape(9), rng.standard_normal(3).astype(np.float32)
+
+
+def gradient_like_systems():
+    """200 (A, b) f64 systems shaped like EstimateColorGradients' normal equations."""
+    rng = np.random.default_rng(9)
+    for _ in range(200):
+        n = rng.normal(size=3)
+        n /= np.linalg.norm(n)
+        P = rng.normal(0, 0.03, (25, 3))
+        P -= np.outer(P @ n, n)                       # tangent-plane offsets
+        A = P.T @ P + 25 * 25 * np.outer(n, n)        # + the orthogonality row (i-1)^2 n n^T
+        yield A, P.T @ rng.normal(0, 0.1, 25)
+
+
+def huber_residuals():
+    rng = np.random.default_rng(4)
+    return np.concatenate([rng.normal(0, 0.05, 300), rng.normal(0, 2.0, 100), [0.0, 0.05, -0.05, 1.0, -1.0, 1.5]])
+
+
+def odometry_inputs():
+    from tests.synth import PRIMESENSE_K, camera_pose, render_depth
+    Ta, Tb = camera_pose(100), camera_pose(103)
+    da, db = render_depth(Ta).numpy(), render_depth(Tb).numpy()
+    da[40:60, 100:140] = 0            # holes -> NaN after ClipTransform
+    db[300:330, 200:260] = 0
+    return da, db, np.linalg.inv(Ta) @ Tb, np.ascontiguousarray(PRIMESENSE_K, dtype=np.float64)
+
+
+def odometry_level(down):
+    """Source / target vertex maps and target normals of pyramid level `down` (1 = 320x240), and a pose that is not
+    yet aligned: both inliers and truncated outliers."""
+    da, db, T_gt, K = odometry_inputs()
+    ds, dt = oracle.clip_transform(db), oracle.clip_transform(da)
+    Kp = K.copy()
+    for _ in range(down):
+        ds, dt = oracle.pyr_down_depth(ds, 0.14), oracle.pyr_down_depth(dt, 0.14)
+        Kp = Kp / 2
+        Kp[2, 2] = 1
+    sv, tv = oracle.create_vertex_map(ds, Kp), oracle.create_vertex_map(dt, Kp)
+    tn = oracle.create_normal_map(oracle.create_vertex_map(oracle.filter_bilateral(dt), Kp))
+    T = T_gt.copy()
+    T[:3, 3] += [0.01, -0.02, 0.015]
+    return sv, tv, tn, Kp, T
+
+
+def color_gradient_clusters():
+    """80 (surface, points, normals, colours) clusters: well-conditioned blobs and thin surface patches."""
+    rng = np.random.default_rng(11)
+    for trial in range(80):
+        surface = trial % 2 == 1
+        k = int(rng.integers(5, 9)) if not surface else int(rng.integers(12, 31))
+        nrm1 = rng.normal(size=3)
+        nrm1 /= np.linalg.norm(nrm1)
+        pts = rng.normal(0, 0.6, (k, 3))
+        if surface:                                     # a thin patch: tangent offsets 3 cm, 1 mm off-plane noise
+            pts = rng.normal(0, 0.03, (k, 3))
+            pts -= np.outer(pts @ nrm1, nrm1) * 0.97
+        pts = pts.astype(np.float32)
+        yield surface, pts, np.tile(nrm1.astype(np.float32), (k, 1)), rng.uniform(0, 1, (k, 3)).astype(np.float32)
+
+
+def tiny_cluster():
+    pts = np.float32([[0, 0, 0], [0.1, 0, 0], [0, 0.1, 0]])
+    return pts, np.tile(np.float32([0, 0, 1]), (3, 1)), np.float32([[0.1] * 3, [0.5] * 3, [0.9] * 3])
+
+
+def information_matrix_inputs():
+    from tests.synth import make_icp_pair
+    src, tgt, _, T = make_icp_pair(6000, seed=3)
+    idx, _, _ = oracle.hybrid_search(tgt, oracle.transform_points(T, src), 0.05, 1)
+    corr = np.ascontiguousarray(idx[:, 0], np.int64)
+    corr[::7] = -1
+    return tgt, corr
+
+
+# ------------------------------------------------ tests
+
+def test_hashes(ref):
+    keys, cells, points = hash_inputs()
+    ref.check("minivec_hash", oracle.minivec_hash(keys).astype(np.uint64))
+    ref.check("spatial_hash", oracle.spatial_hash(cells).astype(np.uint64))
+    ref.check("voxel_index", np.array([oracle.compute_voxel_index(np.array(p, np.float32), inv) for p, inv in points],
+                                      np.int32))
+
+
+def test_robust_kernel_weights_bit_exact(ref):
+    w64, w32 = ref["robust_weight_f64"], ref["robust_weight_f32"]
+    for method in range(7):
+        for i, scale in enumerate(ROBUST_SCALES):
+            for j, shape in enumerate(ROBUST_SHAPES):
+                for k, r in enumerate(ROBUST_RS):
+                    assert oracle.robust_weight(method, scale, shape, r) == w64[method, i, j, k]
+                    a = oracle.robust_weight(method, scale, shape, r, f32=True)
+                    b = w32[method, i, j, k]
+                    assert np.float32(a).tobytes() == b.tobytes(), (method, scale, shape, r, a, b)
+
+
+def test_jacobian_and_sums_bit_exact(ref):
+    """The 29 sums re-accumulated in f32, in index order, from the REFERENCE's Jacobian function."""
+    src, tgt, nrm, corr = p2plane_inputs()
+    ref.check("p2plane_jacobian_sums32", oracle.pose_p2plane_sums(src, tgt, nrm, corr)["sums32"])
+
+
+def test_colored_jacobian_bit_exact(ref):
+    src, sc, tgt, nrm, tc, grad, corr, lam = colored_inputs()
+    ref.check("colored_jacobian_sums64", oracle.pose_colored_sums(src, sc, tgt, nrm, tc, grad, corr, lam)["sums64"])
+
+
+def test_pose_transform_and_indexers_bit_exact(ref):
+    poses, T, pts = pose_inputs()
+    ref.check("pose_to_transformation", np.stack([oracle.pose_to_transformation(p).ravel() for p in poses]))
+    ref.check("transform_points", oracle.transform_points(T, pts))
+    ref.check("transform_normals", oracle.transform_normals(T, pts))
+    # ArrayIndexer conventions the TSDF oracle relies on
+    want = np.concatenate([[[w % res, (w // res) % res, w // (res * res)] for w in range(0, res ** 3, 7)]
+                           for res in (2, 8, 16)]).astype(np.int32)
+    ref.check("workload_to_coord3", want)
+    want = [bool(y >= 0 and x >= 0 and y <= 480 - 1.0 and x <= 640 - 1.0) for x, y in BOUNDARY_POINTS]
+    ref.check("in_boundary2", np.array(want))
+
+
+def test_tsdf_geometry_against_transform_indexer(ref):
+    """One voxel of oracle.tsdf_integrate re-derived with the reference's TransformIndexer (voxel -> camera -> pixel)
+    and InBoundary."""
+    _, _, depth, tsdf, wt, samples = tsdf_geometry_inputs()
+    cams, uvs, inside = ref["indexer_cam"], ref["indexer_uv"], ref["indexer_in_boundary"]
+    checked = 0
+    trunc = np.float32(0.008) * np.float32(8.0)
+    for (b, v, _), cam, uv, inb in zip(samples, cams, uvs, inside):
+        u, vv = uv[0], uv[1]
+        if not inb:
+            assert wt[b, v] == 0
+            continue
+        d = np.float32(depth[int(vv), int(u)]) / np.float32(1000.0)
+        sdf = np.float32(d - cam[2])
+        if d <= 0 or d > 3.0 or cam[2] <= 0 or sdf < -trunc:
+            assert wt[b, v] == 0
+            continue
+        sdf = np.float32(min(sdf, trunc)) / trunc
+        assert wt[b, v] == 1 and np.float32(tsdf[b, v]).tobytes() == np.float32((np.float32(0) * np.float32(0) + sdf) * np.float32(1.0)).tobytes()
+        checked += 1
+    assert checked > 50
+
+
+def test_svd3_solver_bit_exact_vs_reference(ref):
+    """oracle/svd3_oracle.c (svd3x3<float> + solve_svd3x3<float> restated, indexed by axis triples) vs the
+    reference's own solve_svd3x3<float> (core/linalg/kernel/SVD3x3.h:2170-2215) compiled unmodified in oracle/_ref:
+    identical BYTES on general, symmetric-PSD, colour-gradient-like (condition ~1e5), diagonal/scaled, rank-1
+    single-entry and all-zero systems — every branch of the approximate Givens, the column sort and the QR."""
+    ref.check("solve_svd3x3_f32", np.array([oracle.solve_svd3x3(A32, b32) for _, A32, b32 in svd3_systems()]))
     # and the decomposition is what it claims on a benign matrix: A ~= U diag(S) V^T, S sorted by magnitude
     A = np.float32([[2, 0.5, 0.1], [0.5, 1.5, 0.2], [0.1, 0.2, 1.0]])
     U, S, V = oracle.svd3x3(A)
@@ -240,29 +268,22 @@ def test_sym3x3_pinv_vs_reference_svd_solver(ref):
     The reference's Float32 instantiation runs a 4-sweep approximate Jacobi (rsqrt-based Givens), which on
     these systems is NOT an accurate solver: measured here median ~12 %, max ~66 % away from the exact
     solution, while the exact solve of the SAME f32-rounded inputs moves by ~1e-4.  The product's DEFAULT solver
-    reproduces the reference's solve_svd3x3 bit for bit (test_svd3_solver_bit_exact_vs_reference below); the exact
+    reproduces the reference's solve_svd3x3 bit for bit (test_svd3_solver_bit_exact_vs_reference above); the exact
     pseudo-inverse is the opt-in "exact" solver.  This test pins why the option exists: the oracle's exact solve
     has residual ~0, the reference's solver does not."""
-    ref.ref_solve_svd3x3_f32.argtypes = [f32p, f32p, f32p]
-    rng = np.random.default_rng(9)
+    ref_x32 = ref["gradient_like_solve_svd3x3_f32"]
     dev_ref, dev_round, res_orc, res_ref = [], [], [], []
-    for _ in range(200):
-        n = rng.normal(size=3)
-        n /= np.linalg.norm(n)
-        P = rng.normal(0, 0.03, (25, 3))
-        P -= np.outer(P @ n, n)                       # tangent-plane offsets
-        A = P.T @ P + 25 * 25 * np.outer(n, n)        # + the orthogonality row (i-1)^2 n n^T
-        b = P.T @ rng.normal(0, 0.1, 25)
+    for (A, b), x32 in zip(gradient_like_systems(), ref_x32):
         x = oracle.solve_sym3x3_pinv(A, b)
         np.testing.assert_allclose(x, np.linalg.solve(A, b), rtol=1e-9, atol=1e-12)
-        A32, b32, x32 = A.ravel().astype(np.float32), b.astype(np.float32), np.zeros(3, np.float32)
-        ref.ref_solve_svd3x3_f32(_p(A32, f32p), _p(b32, f32p), _p(x32, f32p))
+        A32, b32 = A.ravel().astype(np.float32), b.astype(np.float32)
         scale = np.abs(x).max() + 1e-12
         dev_ref.append(float(np.abs(x32 - x).max() / scale))
         xr = oracle.solve_sym3x3_pinv(A32.astype(np.float64).reshape(3, 3), b32.astype(np.float64))
         dev_round.append(float(np.abs(xr - x).max() / scale))
         res_orc.append(float(np.linalg.norm(A @ x - b) / np.linalg.norm(b)))
         res_ref.append(float(np.linalg.norm(A @ x32.astype(np.float64) - b) / np.linalg.norm(b)))
+    assert len(dev_ref) == 200
     assert max(res_orc) < 1e-10                       # the oracle solves the system
     assert max(dev_round) < 5e-3                      # f32 input rounding alone is harmless
     assert np.all(np.isfinite(dev_ref))
@@ -273,120 +294,63 @@ def test_sym3x3_pinv_vs_reference_svd_solver(ref):
 
 # ------------------------------------------------ RGB-D odometry + image pyramid (SURVEY 8f #2)
 
-def _odometry_inputs(level_div=4):
-    from tests.synth import PRIMESENSE_K, camera_pose, render_depth
-    Ta, Tb = camera_pose(100), camera_pose(103)
-    da, db = render_depth(Ta).numpy(), render_depth(Tb).numpy()
-    da[40:60, 100:140] = 0            # holes -> NaN after ClipTransform
-    db[300:330, 200:260] = 0
-    return da, db, np.linalg.inv(Ta) @ Tb, np.ascontiguousarray(PRIMESENSE_K, dtype=np.float64)
-
-
-def _same(a, b):
-    a, b = np.ascontiguousarray(a), np.ascontiguousarray(b)
-    nan = np.isnan(a)
-    return a.shape == b.shape and np.array_equal(nan, np.isnan(b)) and \
-        np.array_equal(a[~nan].view(np.uint32), b[~nan].view(np.uint32))
-
-
 def test_image_pyramid_kernels_match_reference_functions(ref):
     """ClipTransformCPU, PyrDownDepthCPU, CreateVertexMapCPU, CreateNormalMapCPU compiled from
-    t/geometry/kernel/ImageImpl.h:86-315 (whole functions, NaN fills) vs the oracle: bit-exact."""
-    vp = C.c_void_p
-    ref.ref_clip_transform.argtypes = [vp, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float, f32p]
-    ref.ref_pyr_down_depth.argtypes = [f32p, C.c_int, C.c_int, C.c_float, C.c_float, f32p]
-    ref.ref_create_vertex_map.argtypes = [f32p, C.c_int, C.c_int, f64p, C.c_float, f32p]
-    ref.ref_create_normal_map.argtypes = [f32p, C.c_int, C.c_int, C.c_float, f32p]
-    da, _, _, K = _odometry_inputs()
+    t/geometry/kernel/ImageImpl.h:86-315 (whole functions, NaN fills) vs the oracle: bit-exact, NaN where NaN."""
+    da, _, _, K = odometry_inputs()
     rows, cols = da.shape
     nan = float("nan")
     for src, is_f32 in ((da, 0), ((da.astype(np.float32) / 1000.0), 1)):
-        src = np.ascontiguousarray(src)
-        want = np.empty((rows, cols), np.float32)
         scale = 1000.0 if not is_f32 else 1.0
-        ref.ref_clip_transform(src.ctypes.data, is_f32, rows, cols, scale, 0.0, 3.0, nan, _p(want, f32p))
-        got = oracle.clip_transform(src, scale, 0.0, 3.0, nan)
-        assert np.isnan(got).any() and _same(got, want)
+        got = oracle.clip_transform(np.ascontiguousarray(src), scale, 0.0, 3.0, nan)
+        assert np.isnan(got).any()
+        ref.check(f"clip_transform_{is_f32}", got)
     depth = oracle.clip_transform(da)
-    r, c = rows, cols
     Kp = K.copy()
     for level in range(3):
-        v_want = np.empty((r, c, 3), np.float32)
-        ref.ref_create_vertex_map(_p(depth, f32p), r, c, _p(Kp.reshape(9), f64p), nan, _p(v_want, f32p))
         v_got = oracle.create_vertex_map(depth, Kp)
-        assert _same(v_got, v_want)
-        n_want = np.empty((r, c, 3), np.float32)
-        ref.ref_create_normal_map(_p(v_want, f32p), r, c, nan, _p(n_want, f32p))
-        assert _same(oracle.create_normal_map(v_got), n_want)
-        d_want = np.empty((r // 2, c // 2), np.float32)
-        ref.ref_pyr_down_depth(_p(depth, f32p), r, c, 0.14, nan, _p(d_want, f32p))
+        ref.check(f"vertex_map_{level}", v_got)
+        ref.check(f"normal_map_{level}", oracle.create_normal_map(v_got))
         depth = oracle.pyr_down_depth(depth, 0.14)
-        assert _same(depth, d_want) and np.isnan(depth).any() and np.isfinite(depth).mean() > 0.9
-        r, c = r // 2, c // 2
+        ref.check(f"pyr_down_depth_{level}", depth)
+        assert np.isnan(depth).any() and np.isfinite(depth).mean() > 0.9
         Kp = Kp / 2
         Kp[2, 2] = 1
     # a finite invalid_fill exercises the == branches of PyrDownDepth / CreateNormalMap / is_invalid
     d0 = np.where(np.isnan(oracle.clip_transform(da)), np.float32(0), oracle.clip_transform(da))
-    v_want = np.empty((rows, cols, 3), np.float32)
-    ref.ref_create_vertex_map(_p(d0, f32p), rows, cols, _p(K.reshape(9), f64p), 0.0, _p(v_want, f32p))
-    assert _same(oracle.create_vertex_map(d0, K, 0.0), v_want)
-    n_want = np.empty((rows, cols, 3), np.float32)
-    ref.ref_create_normal_map(_p(v_want, f32p), rows, cols, 0.0, _p(n_want, f32p))
-    assert _same(oracle.create_normal_map(v_want, 0.0), n_want)
-    p_want = np.empty((rows // 2, cols // 2), np.float32)
-    ref.ref_pyr_down_depth(_p(d0, f32p), rows, cols, 0.14, 0.0, _p(p_want, f32p))
-    assert _same(oracle.pyr_down_depth(d0, 0.14, 0.0), p_want)
+    v0 = oracle.create_vertex_map(d0, K, 0.0)
+    ref.check("vertex_map_fill0", v0)
+    ref.check("normal_map_fill0", oracle.create_normal_map(v0, 0.0))
+    ref.check("pyr_down_depth_fill0", oracle.pyr_down_depth(d0, 0.14, 0.0))
 
 
 def test_odometry_huber_and_jacobian_match_reference_header(ref):
     """RGBDOdometryJacobianImpl.h:29-37 (HuberDeriv truncates the residual to int inside Sign()) and
     :106-160 GetJacobianPointToPlane, every pixel of a 120x160 level."""
-    ref.ref_huber_deriv.restype = C.c_float
-    ref.ref_huber_deriv.argtypes = [C.c_float, C.c_float]
-    ref.ref_huber_loss.restype = C.c_float
-    ref.ref_huber_loss.argtypes = [C.c_float, C.c_float]
-    ref.ref_odometry_jacobian_p2plane.argtypes = [C.c_int, C.c_int, C.c_float, f32p, f32p, f32p, C.c_int, C.c_int,
-                                                  f64p, f64p, f32p, f32p]
-    rng = np.random.default_rng(4)
-    for r in np.concatenate([rng.normal(0, 0.05, 300), rng.normal(0, 2.0, 100), [0.0, 0.05, -0.05, 1.0, -1.0, 1.5]]):
-        for delta in (0.05, 0.1, 1.2):
-            a, b = np.float32(oracle.huber_deriv(r, delta)), np.float32(ref.ref_huber_deriv(r, delta))
-            assert a.view(np.uint32) == b.view(np.uint32), (r, delta)
-            a, b = np.float32(oracle.huber_loss(r, delta)), np.float32(ref.ref_huber_loss(r, delta))
-            assert a.view(np.uint32) == b.view(np.uint32), (r, delta)
+    rs = huber_residuals()
+    ref.check("huber_deriv", np.float32([[oracle.huber_deriv(r, d) for d in HUBER_DELTAS] for r in rs]))
+    ref.check("huber_loss", np.float32([[oracle.huber_loss(r, d) for d in HUBER_DELTAS] for r in rs]))
     assert oracle.huber_deriv(0.06, 0.05) == 0.0 and oracle.huber_deriv(1.5, 0.05) == np.float32(0.05)   # the int Sign()
-    da, db, T_gt, K = _odometry_inputs()
-    ds, dt = oracle.clip_transform(db), oracle.clip_transform(da)
-    Kp = K.copy()
-    for _ in range(2):
-        ds, dt = oracle.pyr_down_depth(ds, 0.14), oracle.pyr_down_depth(dt, 0.14)
-        Kp = Kp / 2
-        Kp[2, 2] = 1
-    sv, tv = oracle.create_vertex_map(ds, Kp), oracle.create_vertex_map(dt, Kp)
-    tn = oracle.create_normal_map(oracle.create_vertex_map(oracle.filter_bilateral(dt), Kp))
-    rows, cols = ds.shape
-    T = T_gt.copy()
-    T[:3, 3] += [0.01, -0.02, 0.015]     # not yet aligned: both inliers and truncated outliers
-    Kf, Tf = np.ascontiguousarray(Kp.reshape(9)), np.ascontiguousarray(T.reshape(16))
-    J, r = np.zeros(6, np.float32), np.zeros(1, np.float32)
-    valid = 0
+    sv, tv, tn, Kp, T = odometry_level(2)
+    rows, cols = sv.shape[:2]
+    ok = np.zeros((rows, cols), bool)
+    J = np.zeros((rows, cols, 6), np.float32)
+    r = np.zeros((rows, cols), np.float32)
     for y in range(rows):
         for x in range(cols):
-            ok = ref.ref_odometry_jacobian_p2plane(x, y, 0.07, _p(sv, f32p), _p(tv, f32p), _p(tn, f32p), rows, cols,
-                                                   _p(Kf, f64p), _p(Tf, f64p), _p(J, f32p), _p(r, f32p))
-            ok2, J2, r2 = oracle.odometry_jacobian_p2plane(x, y, sv, tv, tn, Kp, T, 0.07)
-            assert bool(ok) == ok2
-            if ok:
-                valid += 1
-                assert np.array_equal(J.view(np.uint32), J2.view(np.uint32))
-                assert np.float32(r[0]).view(np.uint32) == np.float32(r2).view(np.uint32)
-    assert 0.3 * rows * cols < valid < rows * cols
+            ok[y, x], J2, r2 = oracle.odometry_jacobian_p2plane(x, y, sv, tv, tn, Kp, T, 0.07)
+            if ok[y, x]:
+                J[y, x], r[y, x] = J2, r2
+    ref.check("odometry_jacobian_valid", ok)
+    ref.check("odometry_jacobian_J", J)
+    ref.check("odometry_jacobian_r", r)
+    assert 0.3 * rows * cols < ok.sum() < rows * cols
 
 
 # ------------------------------------------------ whole CPU reduction kernels of the reference (ref_shim_reg.cpp)
 
 def _check_sums(got64, abs64, want, rtol=2e-5):
-    """the reference accumulates Float32 terms in f32 (serially here, ~6 k terms: its own rounding noise is
+    """the reference accumulates Float32 terms in f32 (serially, ~6 k terms: its own rounding noise is
     ~sqrt(n) eps = 5e-6 of sum|term|, measured 3e-6); the oracle accumulates the same f32 terms in f64: equal inlier
     count, every slot within rtol * sum|term|"""
     want = np.asarray(want)
@@ -395,51 +359,28 @@ def _check_sums(got64, abs64, want, rtol=2e-5):
     assert (err <= rtol * abs64 + 1e-12).all(), (err / (abs64 + 1e-300)).max()
 
 
-@pytest.mark.parametrize("robust", [("L2Loss", 1.0, 1.0), ("L1Loss", 1.0, 1.0), ("HuberLoss", 0.01, 1.0),
-                                    ("TukeyLoss", 0.03, 1.0), ("GeneralizedLoss", 0.5, 1.3)])
+@pytest.mark.parametrize("robust", ROBUST)
 def test_pose_sums_match_reference_cpu_kernels(ref, robust):
     """ComputePosePointToPlaneCPU and ComputePoseColoredICPCPU (t/pipelines/kernel/RegistrationCPU.cpp:30-218) as
     whole functions — Jacobian, robust weight dispatch, slot layout, residual / count slots."""
     from tests.synth import make_colors, make_icp_pair
-    ref.ref_pose_p2plane_sums_f32.argtypes = [f32p, f32p, f32p, i64p, C.c_int64, C.c_int64, C.c_int, C.c_double,
-                                              C.c_double, f64p]
-    ref.ref_pose_colored_sums_f32.argtypes = [f32p] * 6 + [i64p, C.c_int64, C.c_int64, C.c_int, C.c_double, C.c_double,
-                                                           C.c_double, f64p]
     src, tgt, nrm, _ = make_icp_pair(6000, seed=12)
     idx, _, _ = oracle.hybrid_search(tgt, src, 0.05, 1)
     corr = np.ascontiguousarray(idx[:, 0].astype(np.int64))
-    method = oracle.ROBUST[robust[0]]
-    want = np.zeros(29)
-    ref.ref_pose_p2plane_sums_f32(_p(src, f32p), _p(tgt, f32p), _p(nrm, f32p), _p(corr, i64p), len(src), len(tgt),
-                                  method, robust[1], robust[2], _p(want, f64p))
     o = oracle.pose_p2plane_sums(src, tgt, nrm, corr, robust)
-    _check_sums(o["sums64"], o["abs64"], want)
+    _check_sums(o["sums64"], o["abs64"], ref[f"pose_p2plane_sums_{robust[0]}"])
     sc, tc = make_colors(src, 1), make_colors(tgt, 1)
     grad = np.ascontiguousarray(np.random.default_rng(1).normal(0, 0.5, tgt.shape).astype(np.float32))
-    ref.ref_pose_colored_sums_f32(_p(src, f32p), _p(sc, f32p), _p(tgt, f32p), _p(nrm, f32p), _p(tc, f32p), _p(grad, f32p),
-                                  _p(corr, i64p), len(src), len(tgt), method, robust[1], robust[2], 0.968, _p(want, f64p))
     o = oracle.pose_colored_sums(src, sc, tgt, nrm, tc, grad, corr, 0.968, robust)
-    _check_sums(o["sums64"], o["abs64"], want)
+    _check_sums(o["sums64"], o["abs64"], ref[f"pose_colored_sums_{robust[0]}"])
 
 
 def test_odometry_sums_match_reference_cpu_kernel(ref):
     """odometry::ComputeOdometryResultPointToPlaneCPU (t/pipelines/kernel/RGBDOdometryCPU.cpp:286-362) as a whole
     function on a 240x320 level."""
-    ref.ref_odometry_p2plane_sums.argtypes = [f32p, f32p, f32p, C.c_int, C.c_int, f64p, f64p, C.c_float, C.c_float, f64p]
-    da, db, T_gt, K = _odometry_inputs()
-    ds, dt = oracle.pyr_down_depth(oracle.clip_transform(db), 0.14), oracle.pyr_down_depth(oracle.clip_transform(da), 0.14)
-    Kp = K / 2
-    Kp[2, 2] = 1
-    sv, tv = oracle.create_vertex_map(ds, Kp), oracle.create_vertex_map(dt, Kp)
-    tn = oracle.create_normal_map(oracle.create_vertex_map(oracle.filter_bilateral(dt), Kp))
-    T = T_gt.copy()
-    T[:3, 3] += [0.01, -0.02, 0.015]
-    want = np.zeros(29)
-    Kf, Tf = np.ascontiguousarray(Kp.reshape(9)), np.ascontiguousarray(T.reshape(16))
-    ref.ref_odometry_p2plane_sums(_p(sv, f32p), _p(tv, f32p), _p(tn, f32p), sv.shape[0], sv.shape[1], _p(Kf, f64p),
-                                  _p(Tf, f64p), 0.07, 0.05, _p(want, f64p))
+    sv, tv, tn, Kp, T = odometry_level(1)
     o = oracle.odometry_p2plane_sums(sv, tv, tn, Kp, T, 0.07, 0.05)
-    _check_sums(o["sums64"], o["abs64"], want, rtol=1e-4)   # ~70 k f32 terms upstream
+    _check_sums(o["sums64"], o["abs64"], ref["odometry_p2plane_sums"], rtol=1e-4)   # ~70 k f32 terms upstream
 
 
 def test_color_gradient_kernel_bit_exact_vs_reference_kernel(ref):
@@ -449,57 +390,33 @@ def test_color_gradient_kernel_bit_exact_vs_reference_kernel(ref):
     row, the f32 normal equations and the reference's 4-sweep SVD solve — on well-conditioned clusters and on
     surface-like neighbourhoods (condition ~1e5, where the fast SVD is far from the exact solution).  The "exact"
     solver option differs from the reference there, by design (last assertion)."""
-    ref.ref_color_gradient_point_f32.argtypes = [f32p, f32p, f32p, C.c_int64, i32p, C.c_int32, f32p]
-    rng = np.random.default_rng(11)
+    want_all = ref["color_gradients"]
     gap = []
-    for trial in range(80):
-        surface = trial % 2 == 1
-        k = int(rng.integers(5, 9)) if not surface else int(rng.integers(12, 31))
-        nrm1 = rng.normal(size=3)
-        nrm1 /= np.linalg.norm(nrm1)
-        pts = rng.normal(0, 0.6, (k, 3))
-        if surface:                                     # a thin patch: tangent offsets 3 cm, 1 mm off-plane noise
-            pts = rng.normal(0, 0.03, (k, 3))
-            pts -= np.outer(pts @ nrm1, nrm1) * 0.97
-        pts = pts.astype(np.float32)
-        nrm = np.tile(nrm1.astype(np.float32), (k, 1))
-        col = rng.uniform(0, 1, (k, 3)).astype(np.float32)
+    at = 0
+    for trial, (surface, pts, nrm, col) in enumerate(color_gradient_clusters()):
+        k = len(pts)
         got = oracle.estimate_color_gradients(pts, nrm, col, 10.0, 30)            # every point sees the whole cluster
         exact = oracle.estimate_color_gradients(pts, nrm, col, 10.0, 30, solver="exact")
         idx, _, cnt = oracle.hybrid_search(pts, pts, 10.0, 30)
         assert (cnt == k).all() and (idx[:, 0] == np.arange(k)).all()
-        want = np.full_like(pts, 7.0)
-        for i in range(k):
-            row = np.ascontiguousarray(idx[i], np.int32)
-            ref.ref_color_gradient_point_f32(_p(pts, f32p), _p(nrm, f32p), _p(col, f32p), i, _p(row, i32p), int(cnt[i]),
-                                             _p(want, f32p))
+        want = want_all[at:at + k]
+        at += k
         assert got.tobytes() == want.tobytes(), (trial, np.abs(got - want).max())
         if surface:
             gap.append(float(np.abs(exact - want).max() / (np.abs(exact).max() + 1e-12)))
+    assert at == len(want_all)
     assert np.median(gap) > 1e-3, np.median(gap)       # the exact option is NOT the reference's result on such systems
     # fewer than 4 neighbours: exactly zero on both sides
-    pts = np.float32([[0, 0, 0], [0.1, 0, 0], [0, 0.1, 0]])
-    nrm = np.tile(np.float32([0, 0, 1]), (3, 1))
-    col = np.float32([[0.1] * 3, [0.5] * 3, [0.9] * 3])
-    want = np.full_like(pts, 7.0)
-    row = np.int32([0, 1, 2])
-    ref.ref_color_gradient_point_f32(_p(pts, f32p), _p(nrm, f32p), _p(col, f32p), 0, _p(row, i32p), 3, _p(want, f32p))
-    assert not want[0].any() and not oracle.estimate_color_gradients(pts, nrm, col, 1.0, 30).any()
+    want = ref["color_gradient_three_neighbours"]
+    assert not want.any() and not oracle.estimate_color_gradients(*tiny_cluster(), 1.0, 30).any()
 
 
 def test_information_matrix_matches_reference_cpu_kernel(ref):
     """ComputeInformationMatrixCPU (t/pipelines/kernel/RegistrationCPU.cpp:655-735, compiled unmodified; its
     tbb::parallel_reduce runs as one serial f32 pass in the shim) vs the oracle's GTG (same f32 terms, f64 sums):
     equal to the rounding noise of the reference's own f32 accumulation, unmatched points (-1) skipped on both sides."""
-    from tests.synth import make_icp_pair
-    ref.ref_information_matrix_f32.argtypes = [f32p, C.c_int64, i64p, C.c_int64, f64p]
-    src, tgt, _, T = make_icp_pair(6000, seed=3)
-    idx, _, _ = oracle.hybrid_search(tgt, oracle.transform_points(T, src), 0.05, 1)
-    corr = np.ascontiguousarray(idx[:, 0], np.int64)
-    corr[::7] = -1
-    want = np.zeros(36)
-    ref.ref_information_matrix_f32(_p(tgt, f32p), len(tgt), _p(corr, i64p), len(corr), _p(want, f64p))
-    want = want.reshape(6, 6)
+    tgt, corr = information_matrix_inputs()
+    want = ref["information_matrix"].reshape(6, 6)
     got = oracle.information_matrix(tgt, corr)
     assert np.array_equal(got, got.T) and np.array_equal(want, want.T)
     n_valid = int((corr >= 0).sum())

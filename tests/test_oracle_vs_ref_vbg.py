@@ -1,55 +1,34 @@
-"""The oracle's voxel-block-grid path against the reference's OWN CPU implementation: oracle/_ref/libo3dref.so contains
-t/geometry/kernel/VoxelBlockGridCPU.cpp + VoxelBlockGridImpl.h compiled unmodified (oracle/ref_shim/ref_shim_vbg.cpp,
-stub Tensor/HashMap/TBB headers, serial ParallelFor): DepthTouchCPU, IntegrateCPU, EstimateRangeCPU, RayCastCPU as whole
-functions.  Every comparison is bit-exact.  CPU only."""
-import ctypes as C
-import os
+"""The oracle's voxel-block-grid path against the reference's OWN CPU implementation: t/geometry/kernel/
+VoxelBlockGridCPU.cpp + VoxelBlockGridImpl.h compiled unmodified (oracle/ref_shim/ref_shim_vbg.cpp, stub
+Tensor/HashMap/TBB headers, serial ParallelFor): what DepthTouchCPU, IntegrateCPU, EstimateRangeCPU and RayCastCPU
+return on the inputs built here, stored in tests/golden/ref_oracle_vs_ref_vbg.npz by tests/golden/make_ref_vectors.py.
+Every comparison is bit-exact.  CPU only."""
+import functools
 
 import numpy as np
 import pytest
 
 import oracle
+from tests.ref_vectors import Vectors
 from tests.synth import PRIMESENSE_K, camera_pose, render_depth
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "oracle", "_ref", "libo3dref.so")
-pytestmark = pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref not built (needs /root/reference)")
 
 VOXEL, RES, TRUNC = 0.008, 16, 8.0
 SCALE, DMIN, DMAX = 1000.0, 0.1, 3.0
-f32p, f64p, i32p = C.POINTER(C.c_float), C.POINTER(C.c_double), C.POINTER(C.c_int32)
-vp = C.c_void_p
-
-
-def _p(a, t):
-    return a.ctypes.data_as(t)
+K9 = np.ascontiguousarray(np.asarray(PRIMESENSE_K, np.float64).reshape(9))
+DEPTH_TOUCH_FRAMES = [(0, False), (137, False), (500, True)]
+VOLUME_FRAMES, VOLUME_CAPACITY = (100, 102, 104, 106), 4000
+RANGE_DOWN = [8, 4]
+RAY_CAST_VIEWS = [(106, 3.0), (103, 1.0), (140, 1.0)]
+RAY_CAST_ATTRS = ("depth", "vertex", "color", "normal", "index", "mask", "interp_ratio", "interp_ratio_dx",
+                  "interp_ratio_dy", "interp_ratio_dz")
 
 
 @pytest.fixture(scope="module")
 def ref():
-    L = C.CDLL(REF)
-    L.ref_depth_touch.restype = C.c_int64
-    L.ref_depth_touch.argtypes = [vp, C.c_int, C.c_int, C.c_int, f64p, f64p, C.c_int, C.c_float, C.c_float, C.c_float,
-                                  C.c_float, C.c_int, i32p, C.c_int64]
-    L.ref_integrate_f32_values.restype = None
-    L.ref_integrate_f32_values.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, i32p, C.c_int64, i32p, C.c_int64, f32p, vp, vp, f64p,
-                                           f64p, f64p, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float]
-    L.ref_integrate.restype = None
-    L.ref_integrate.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, i32p, C.c_int64, i32p, C.c_int64, f32p, vp, vp, f64p,
-                                f64p, f64p, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float]
-    L.ref_estimate_range.restype = C.c_int64
-    L.ref_estimate_range.argtypes = [i32p, C.c_int64, f64p, f64p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float,
-                                     C.c_float, C.c_float, C.c_int64, f32p]
-    L.ref_ray_cast.restype = None
-    L.ref_ray_cast.argtypes = [i32p, C.c_int64, f32p, vp, vp, f32p, f64p, f64p, C.c_int, C.c_int, C.c_int, C.c_float,
-                               C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_int] + [vp] * 10
-    return L
+    return Vectors("oracle_vs_ref_vbg")
 
 
-K9 = np.ascontiguousarray(np.asarray(PRIMESENSE_K, np.float64).reshape(9))
-
-
-def _frame(i, f32=False):
+def frame(i, f32=False):
     T = camera_pose(i)
     depth, color = render_depth(T, with_color=True)
     depth, color = depth.numpy(), color.numpy()
@@ -58,78 +37,60 @@ def _frame(i, f32=False):
     return oracle.inverse_transformation(T), np.ascontiguousarray(depth), np.ascontiguousarray(color)
 
 
-def _sorted(k):
+def sorted_keys(k):
     k = np.asarray(k, np.int32).reshape(-1, 3)
     return k[np.lexsort((k[:, 2], k[:, 1], k[:, 0]))]
 
 
-@pytest.mark.parametrize("fid,f32", [(0, False), (137, False), (500, True)])
+def fuse(frames, cap, value_dtype=np.uint16, f32_inputs=False, with_color=True):
+    """`frames` fused by the oracle: the hash map's keys and size, tsdf / weight / colour buffers, last frustum."""
+    keys = np.zeros((cap, 3), np.int32)
+    t, w = np.zeros((cap, RES ** 3), np.float32), np.zeros((cap, RES ** 3), value_dtype)
+    col = np.zeros((cap, RES ** 3, 3), value_dtype)
+    size, touched = 0, None
+    for fid in frames:
+        E, depth, color = frame(fid, f32_inputs)
+        touched = oracle.depth_touch(depth, PRIMESENSE_K, E, RES, VOXEL, VOXEL * TRUNC, SCALE, DMAX, 4)
+        bi, _, size, rc = oracle.hashmap_activate(keys, size, touched)
+        assert rc == 0
+        oracle.tsdf_integrate(depth, color if with_color else None, bi, keys, t, w, col if with_color else None,
+                              PRIMESENSE_K, PRIMESENSE_K, E, RES, VOXEL, VOXEL * TRUNC, SCALE, DMAX)
+    return dict(keys=keys, size=size, o=dict(tsdf=t, wt=w, col=col), frustum=touched)
+
+
+@functools.lru_cache(maxsize=1)
+def oracle_volume():
+    """Four colour frames fused by the oracle (the reference's IntegrateCPU fuses the same frames on the same block
+    indices into the stored buffers)."""
+    return fuse(VOLUME_FRAMES, VOLUME_CAPACITY)
+
+
+@pytest.mark.parametrize("fid,f32", DEPTH_TOUCH_FRAMES)
 def test_depth_touch_is_the_reference_block_set(ref, fid, f32):
     """DepthTouchCPU (VoxelBlockGridCPU.cpp:117-201): identical set of touched blocks."""
-    E, depth, _ = _frame(fid, f32)
-    Ef = np.ascontiguousarray(E.reshape(16))
-    out = np.zeros((76800, 3), np.int32)
-    n = ref.ref_depth_touch(depth.ctypes.data, int(f32), 480, 640, _p(K9, f64p), _p(Ef, f64p), RES, VOXEL, VOXEL * TRUNC,
-                            SCALE, DMAX, 4, _p(out, i32p), len(out))
-    want = _sorted(out[:n])
+    E, depth, _ = frame(fid, f32)
     got = oracle.depth_touch(depth, PRIMESENSE_K, E, RES, VOXEL, VOXEL * TRUNC, SCALE, DMAX, 4)
-    assert n > 300 and np.array_equal(got, want)
+    assert len(got) > 300
+    ref.check(f"depth_touch_{fid}_{int(f32)}", np.asarray(got, np.int32))
 
 
-@pytest.fixture(scope="module")
-def volumes(ref):
-    """Four colour frames fused by the oracle and by the reference's IntegrateCPU into separate buffers."""
-    cap = 4000
-    keys = np.zeros((cap, 3), np.int32)
-    o = dict(tsdf=np.zeros((cap, RES ** 3), np.float32), wt=np.zeros((cap, RES ** 3), np.uint16),
-             col=np.zeros((cap, RES ** 3, 3), np.uint16))
-    r = dict(tsdf=np.zeros((cap, RES ** 3), np.float32), wt=np.zeros((cap, RES ** 3), np.uint16),
-             col=np.zeros((cap, RES ** 3, 3), np.uint16))
-    size, want = 0, None
-    frames = (100, 102, 104, 106)
-    for fid in frames:
-        E, depth, color = _frame(fid)
-        want = oracle.depth_touch(depth, PRIMESENSE_K, E, RES, VOXEL, VOXEL * TRUNC, SCALE, DMAX, 4)
-        bi, _, size, rc = oracle.hashmap_activate(keys, size, want)
-        assert rc == 0
-        oracle.tsdf_integrate(depth, color, bi, keys, o["tsdf"], o["wt"], o["col"], PRIMESENSE_K, PRIMESENSE_K, E, RES,
-                              VOXEL, VOXEL * TRUNC, SCALE, DMAX)
-        Ef = np.ascontiguousarray(E.reshape(16))
-        bi = np.ascontiguousarray(bi, np.int32)
-        ref.ref_integrate(depth.ctypes.data, color.ctypes.data, 0, 480, 640, _p(bi, i32p), len(bi), _p(keys, i32p), cap,
-                          _p(r["tsdf"], f32p), r["wt"].ctypes.data, r["col"].ctypes.data, _p(K9, f64p), _p(K9, f64p),
-                          _p(Ef, f64p), RES, VOXEL, VOXEL * TRUNC, SCALE, DMAX)
-    return dict(keys=keys, size=size, o=o, r=r, frustum=want, last=frames[-1])
-
-
-def test_integrate_is_the_reference_integrate(ref, volumes):
+def test_integrate_is_the_reference_integrate(ref):
     """IntegrateCPU<u16,u8,f32,u16,u16> (VoxelBlockGridImpl.h:151-308) over 4 frames: tsdf bit for bit, weights and
     colours equal."""
-    o, r = volumes["o"], volumes["r"]
+    o = oracle_volume()["o"]
     assert (o["wt"] > 0).sum() > 500000
-    assert np.array_equal(o["wt"], r["wt"]) and np.array_equal(o["col"], r["col"])
-    assert np.array_equal(o["tsdf"].view(np.uint32), r["tsdf"].view(np.uint32))
+    ref.check("integrate_weight", o["wt"])
+    ref.check("integrate_color", o["col"])
+    ref.check("integrate_tsdf", o["tsdf"])
 
 
 def test_integrate_float_inputs_and_depth_only(ref):
     """IntegrateCPU<f32,f32,f32,u16,u16> (colour x 255) and the depth-only call (empty colour tensor)."""
-    cap = 3000
     for with_color in (True, False):
-        keys = np.zeros((cap, 3), np.int32)
-        ot, ow, oc = np.zeros((cap, RES ** 3), np.float32), np.zeros((cap, RES ** 3), np.uint16), np.zeros((cap, RES ** 3, 3), np.uint16)
-        rt, rw, rcol = ot.copy(), ow.copy(), oc.copy()
-        E, depth, color = _frame(300, f32=True)
-        want = oracle.depth_touch(depth, PRIMESENSE_K, E, RES, VOXEL, VOXEL * TRUNC, SCALE, DMAX, 4)
-        bi, _, size, _ = oracle.hashmap_activate(keys, 0, want)
-        oracle.tsdf_integrate(depth, color if with_color else None, bi, keys, ot, ow, oc if with_color else None,
-                              PRIMESENSE_K, PRIMESENSE_K, E, RES, VOXEL, VOXEL * TRUNC, SCALE, DMAX)
-        Ef = np.ascontiguousarray(E.reshape(16))
-        bi = np.ascontiguousarray(bi, np.int32)
-        ref.ref_integrate(depth.ctypes.data, color.ctypes.data if with_color else None, 1, 480, 640, _p(bi, i32p), len(bi),
-                          _p(keys, i32p), cap, _p(rt, f32p), rw.ctypes.data, rcol.ctypes.data if with_color else None,
-                          _p(K9, f64p), _p(K9, f64p), _p(Ef, f64p), RES, VOXEL, VOXEL * TRUNC, SCALE, DMAX)
-        assert np.array_equal(ot.view(np.uint32), rt.view(np.uint32)) and np.array_equal(ow, rw)
-        assert np.array_equal(oc, rcol) and (oc.any() == with_color)
+        o = fuse((300,), 3000, f32_inputs=True, with_color=with_color)["o"]
+        for name, key in (("tsdf", "tsdf"), ("weight", "wt"), ("color", "col")):
+            ref.check(f"integrate_f32_inputs_{int(with_color)}_{name}", o[key])
+        assert o["col"].any() == with_color
 
 
 @pytest.mark.parametrize("f32_inputs", [False, True])
@@ -137,82 +98,44 @@ def test_integrate_float32_value_layout_is_the_reference_integrate(ref, f32_inpu
     """The reference's other value layout — IntegrateCPU<u16,u8,f32,float,float> and <f32,f32,f32,float,float>
     (weight Float32, colour Float32, VoxelBlockGridCPU.cpp instantiations) — over 3 fused frames: tsdf, weight and
     colour bit for bit (the float colour is NOT truncated to an integer in this layout)."""
-    cap = 3000
-    keys = np.zeros((cap, 3), np.int32)
-    ot, ow, oc = np.zeros((cap, RES ** 3), np.float32), np.zeros((cap, RES ** 3), np.float32), np.zeros((cap, RES ** 3, 3), np.float32)
-    rt, rw, rcol = ot.copy(), ow.copy(), oc.copy()
-    size = 0
-    for fid in (300, 302, 304):
-        E, depth, color = _frame(fid, f32=f32_inputs)
-        want = oracle.depth_touch(depth, PRIMESENSE_K, E, RES, VOXEL, VOXEL * TRUNC, SCALE, DMAX, 4)
-        bi, _, size, _ = oracle.hashmap_activate(keys, size, want)
-        oracle.tsdf_integrate(depth, color, bi, keys, ot, ow, oc, PRIMESENSE_K, PRIMESENSE_K, E, RES, VOXEL, VOXEL * TRUNC, SCALE, DMAX)
-        Ef = np.ascontiguousarray(E.reshape(16))
-        bi = np.ascontiguousarray(bi, np.int32)
-        ref.ref_integrate_f32_values(depth.ctypes.data, color.ctypes.data, int(f32_inputs), 480, 640, _p(bi, i32p), len(bi),
-                                     _p(keys, i32p), cap, _p(rt, f32p), rw.ctypes.data, rcol.ctypes.data, _p(K9, f64p), _p(K9, f64p),
-                                     _p(Ef, f64p), RES, VOXEL, VOXEL * TRUNC, SCALE, DMAX)
-    assert np.array_equal(ot.view(np.uint32), rt.view(np.uint32)) and np.array_equal(ow.view(np.uint32), rw.view(np.uint32))
-    assert np.array_equal(oc.view(np.uint32), rcol.view(np.uint32))
-    assert ow.max() == 3.0 and (oc != np.floor(oc)).any()
+    o = fuse((300, 302, 304), 3000, np.float32, f32_inputs)["o"]
+    for name, key in (("tsdf", "tsdf"), ("weight", "wt"), ("color", "col")):
+        ref.check(f"integrate_f32_values_{int(f32_inputs)}_{name}", o[key])
+    assert o["wt"].max() == 3.0 and (o["col"] != np.floor(o["col"])).any()
 
 
-@pytest.mark.parametrize("down", [8, 4])
-def test_estimate_range_is_the_reference_range_map(ref, volumes, down):
+@pytest.mark.parametrize("down", RANGE_DOWN)
+def test_estimate_range_is_the_reference_range_map(ref, down):
     """EstimateRangeCPU (VoxelBlockGridImpl.h:310-555) with a fragment buffer that is large enough; and what upstream
     does when it is not (the mode this library does not have)."""
-    E = oracle.inverse_transformation(camera_pose(volumes["last"]))
-    Ef = np.ascontiguousarray(E.reshape(16))
-    keys = np.ascontiguousarray(volumes["frustum"])
-    want = np.zeros((480 // down, 640 // down, 2), np.float32)
-    ref.ref_estimate_range(_p(keys, i32p), len(keys), _p(K9, f64p), _p(Ef, f64p), 480, 640, down, RES, VOXEL, DMIN, DMAX,
-                           1 << 16, _p(want, f32p))
-    got = oracle.estimate_range(keys, PRIMESENSE_K, E, 480, 640, down, RES, VOXEL, DMIN, DMAX)
-    assert (want[..., 0] < want[..., 1]).mean() > 0.9
-    assert np.array_equal(got.view(np.uint32), want.view(np.uint32))
+    vol = oracle_volume()
+    E = oracle.inverse_transformation(camera_pose(VOLUME_FRAMES[-1]))
+    got = oracle.estimate_range(np.ascontiguousarray(vol["frustum"]), PRIMESENSE_K, E, 480, 640, down, RES, VOXEL,
+                                DMIN, DMAX)
+    assert (got[..., 0] < got[..., 1]).mean() > 0.9
+    ref.check(f"estimate_range_{down}", got)
     # upstream's own first-call allocation, h_down*w_down/256/voxel_size fragments (:341-347) ...
-    auto = np.zeros_like(want)
-    n_auto = ref.ref_estimate_range(_p(keys, i32p), len(keys), _p(K9, f64p), _p(Ef, f64p), 480, 640, down, RES, VOXEL,
-                                    DMIN, DMAX, 0, _p(auto, f32p))
-    assert n_auto >= (480 // down) * (640 // down) // 256 / VOXEL - 1 and np.array_equal(auto, want)
+    assert ref[f"estimate_range_{down}_auto_fragments"] >= (480 // down) * (640 // down) // 256 / VOXEL - 1
+    ref.check(f"estimate_range_{down}_auto", got)
     # ... and a buffer that is too small: fragments are dropped, the map is incomplete (warning upstream)
-    small = np.zeros_like(want)
-    ref.ref_estimate_range(_p(keys, i32p), len(keys), _p(K9, f64p), _p(Ef, f64p), 480, 640, down, RES, VOXEL, DMIN, DMAX,
-                           40, _p(small, f32p))
-    assert not np.array_equal(small, want) and ((small[..., 0] < small[..., 1]).sum() < (want[..., 0] < want[..., 1]).sum())
+    small = ref[f"estimate_range_{down}_small"]
+    assert not np.array_equal(small, got) and ((small[..., 0] < small[..., 1]).sum() < (got[..., 0] < got[..., 1]).sum())
 
 
-@pytest.mark.parametrize("fid,threshold", [(106, 3.0), (103, 1.0), (140, 1.0)])
-def test_ray_cast_is_the_reference_ray_cast(ref, volumes, fid, threshold):
+@pytest.mark.parametrize("fid,threshold", RAY_CAST_VIEWS)
+def test_ray_cast_is_the_reference_ray_cast(ref, fid, threshold):
     """RayCastCPU<float, uint16_t, uint16_t> (VoxelBlockGridImpl.h:578-1120), all ten renderings, on the oracle-fused
     volume: bit-exact everywhere.  (The oracle's two clamps — voxel index res-1, range cell — cannot trigger here:
     640x480 is a multiple of the down factor, and a voxel coordinate that rounds up to `resolution` would show up as a
     mismatch.)"""
-    o = volumes["o"]
+    vol = oracle_volume()
+    o = vol["o"]
     E = oracle.inverse_transformation(camera_pose(fid))
-    Ef = np.ascontiguousarray(E.reshape(16))
-    keys = np.ascontiguousarray(volumes["keys"][: volumes["size"]])
+    keys = np.ascontiguousarray(vol["keys"][: vol["size"]])
     rng = oracle.estimate_range(keys, PRIMESENSE_K, E, 480, 640, 8, RES, VOXEL, DMIN, DMAX)
-    attrs = ("depth", "vertex", "color", "normal", "index", "mask", "interp_ratio", "interp_ratio_dx",
-             "interp_ratio_dy", "interp_ratio_dz")
-    got = oracle.ray_cast(volumes["keys"], volumes["size"], o["tsdf"], o["wt"], o["col"], rng, PRIMESENSE_K, E, 480, 640,
-                          attrs, RES, VOXEL, SCALE, DMIN, DMAX, threshold, TRUNC, 8)
-    want = {}
-    ptrs = []
-    for name in attrs:
-        c, dt = oracle.RAYCAST_ATTRS[name]
-        want[name] = np.full((480, 640, c), 77, dt)
-        ptrs.append(want[name].ctypes.data)
-    ref.ref_ray_cast(_p(volumes["keys"], i32p), volumes["size"], _p(o["tsdf"], f32p), o["wt"].ctypes.data,
-                     o["col"].ctypes.data, _p(rng, f32p), _p(K9, f64p), _p(Ef, f64p), 480, 640, RES, VOXEL, SCALE, DMIN,
-                     DMAX, threshold, TRUNC, 8, *ptrs)
-    hit = want["depth"][..., 0] > 0
+    got = oracle.ray_cast(vol["keys"], vol["size"], o["tsdf"], o["wt"], o["col"], rng, PRIMESENSE_K, E, 480, 640,
+                          RAY_CAST_ATTRS, RES, VOXEL, SCALE, DMIN, DMAX, threshold, TRUNC, 8)
+    hit = got["depth"][..., 0] > 0
     assert hit.mean() > (0.5 if fid != 140 else 0.01)
-    for name in attrs:
-        a, b = got[name], want[name]
-        if name == "mask":
-            b = b.astype(bool)
-        if a.dtype == np.float32:
-            assert np.array_equal(a.view(np.uint32), b.view(np.uint32)), name
-        else:
-            assert np.array_equal(a, b), name
+    for name in RAY_CAST_ATTRS:
+        ref.check(f"ray_cast_{fid}_{name}", got[name])
